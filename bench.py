@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: forward point-clouds / second of the SE(3)-Transformer attention hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload = BASELINE.json configs[1] ("cfg2": batch 4, N=1024, dim 512, heads 8, dim_head 64, depth 6, num_degrees 4,
 k-NN 16) per GPU; with N GPUs every rank runs its own batch of 4 clouds (weak scaling, no data-path collective) and the
@@ -12,6 +12,10 @@ returned type-0 features are all-gathered so that every rank holds the whole bat
   roofline: the dominant kernel (fused tcgen05 pairwise kernel): algorithmic FLOPs / CUDA-event time vs measured bf16 peak
   cpu_baseline / --impl reference: the numpy oracle (port of the reference algorithm) timed on the host cores on a
            bounded, width-preserving sample, extrapolated by algorithmic FLOPs (the full workload needs ~79 h on CPU).
+
+--dump-outputs DIR writes what the last timed step returned (the headline arm: the forward's output, all-gathered over the
+ranks; --impl reference: the sampled ConvSE3's output) as DIR/<name>.npy, so that two builds can be compared output for
+output: inputs and weights come from fixed seeds, identical from run to run for the same arguments.
 """
 import argparse
 import json
@@ -91,6 +95,34 @@ def load_peaks():
         return dict(hbm_gbs=p['hbm_gbs'], bf16_burst=p['bf16_tflops'], bf16_sustained=p.get('bf16_tflops_sustained', p['bf16_tflops']),
                     source='measured (MEASURED_PEAKS.json)')
     return dict(hbm_gbs=6650.0, bf16_burst=1590.0, bf16_sustained=1400.0, source='fallback (B200_PROFILING.md)')
+
+
+DUMP_BYTES = 64 << 20
+
+
+def output_arrays(out):
+    """The forward's return value (one tensor, or a dict degree -> tensor) as host arrays named for --dump-outputs."""
+    import numpy as np
+    host = lambda t: t.detach().cpu().numpy() if hasattr(t, 'detach') else np.asarray(t)
+    if isinstance(out, dict):
+        return {f'type{d}': host(t) for d, t in out.items()}
+    return {'out': host(out)}
+
+
+def dump_outputs(arrays, path):
+    """Write every array as path/<name>.npy, float64 kept and anything else as float32.  Past DUMP_BYTES in all, each array
+    keeps the same fraction of its rows (rows = the flattened batch x point axes), drawn once from a fixed seed and kept in
+    order, so that runs of the same arguments still sample the same points."""
+    import numpy as np
+    arrays = {k: (a if a.dtype == np.float64 else a.astype(np.float32)) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            rows = a.reshape(-1, *a.shape[2:]) if a.ndim > 2 else a.reshape(-1)
+            keep = max(1, len(rows) * DUMP_BYTES // total)
+            a = rows[np.sort(np.random.default_rng(0).choice(len(rows), keep, replace=False))]
+        np.save(os.path.join(path, f'{name}.npy'), a)
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -210,6 +242,8 @@ def run_reference(args, wl, rank, world):
     for _ in range(min(args.warmup, 1)):
         sample.run()
     times = [sample.run() for _ in range(args.steps)]
+    if args.dump_outputs:
+        dump_outputs(output_arrays(sample.out), args.dump_outputs)
     sec = sum(times) / len(times)
     value = sample.clouds_per_s(sec)
     desc = sample.desc
@@ -372,12 +406,15 @@ def run_ours(args, wl, rank, local_rank, world):
     ops.PROFILE = []
     if args.profile_range:
         torch.cuda.cudart().cudaProfilerStart()
-    ms_res, _ = timed(lambda: step_resident(dev_inputs), args.steps)
+    ms_res, last_out = timed(lambda: step_resident(dev_inputs), args.steps)
     if args.profile_range:
         torch.cuda.cudart().cudaProfilerStop()
     prof, ops.PROFILE = ops.PROFILE, None
     launches = ops.LAUNCHES - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(output_arrays(last_out), args.dump_outputs)
+    del last_out
 
     kern = {}
     detail = {}
@@ -500,7 +537,11 @@ def main():
     ap.add_argument('--radial-scale', type=float, default=1.0, help='weights-sensitivity experiment: scale RadialFunc.net.0.weight (rougher radial functions, higher rank)')
     ap.add_argument('--cuda-graph', action='store_true', help='replay the forward from a CUDA graph (launch-bound small workloads)')
     ap.add_argument('--profile-range', action='store_true', help='cudaProfilerStart/Stop around the resident timed steps (for ncu --profile-from-start off)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the output of the last timed step as DIR/<name>.npy (float32/float64, '
+                                                          'at most 64 MB in all: a fixed, seeded sample of the points beyond that)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get('RANK', 0))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))

@@ -222,3 +222,23 @@ def test_plan_guard_bounds_the_output_error(radial, monkeypatch):
             f.write(json.dumps(r) + '\n')
     print(rows)
     assert accepted >= 2, rows          # (whether some scale is rejected depends on the weights; rejected ones never return a result)
+
+
+def test_bench_dumps_the_same_outputs_whatever_the_step_count(tmp_path):
+    """bench.py --dump-outputs on the GPU arm: the last timed forward's output, float32, the same for every run of a workload
+    (seeded weights and inputs) whatever --steps is."""
+    import json
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dumps = []
+    for steps in (1, 3):
+        r = subprocess.run([sys.executable, os.path.join(root, 'bench.py'), '--workload', 'cfg1', '--steps', str(steps), '--warmup', '1',
+                            '--no-cpu-baseline', '--dump-outputs', str(tmp_path / str(steps))], capture_output=True, text=True,
+                           timeout=600, cwd=root)
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith('{')][-1])
+        assert line['steps'] == steps
+        dumps.append(np.load(tmp_path / str(steps) / 'out.npy'))
+    assert dumps[0].dtype == np.float32 and dumps[0].shape == (1, 32, 64) and np.isfinite(dumps[0]).all()
+    assert rel_err(dumps[1], dumps[0]) < 1e-6

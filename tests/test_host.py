@@ -371,6 +371,46 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert _run_bench(['--gpus', '2'], env={'RANK': '1', 'LOCAL_RANK': '1', 'WORLD_SIZE': '2'}) == []
 
 
+def test_reference_arm_dumps_the_same_outputs_whatever_the_step_count(tmp_path):
+    """--dump-outputs writes the last timed step's output as float .npy files; the inputs come from fixed seeds, so runs with
+    other step counts write the same arrays."""
+    import numpy as np
+    dumps = []
+    for steps in (1, 2):
+        (line,) = _run_bench(['--steps', str(steps), '--dump-outputs', str(tmp_path / str(steps))])
+        assert line['steps'] == steps
+        dumps.append({f: np.load(tmp_path / str(steps) / f) for f in sorted(os.listdir(tmp_path / str(steps)))})
+    assert sorted(dumps[0]) == ['type0.npy', 'type1.npy']
+    for f, a in dumps[0].items():
+        assert a.dtype in (np.float32, np.float64) and np.isfinite(a).all() and np.abs(a).max() > 0
+        np.testing.assert_allclose(dumps[1][f], a, rtol=1e-5, atol=0)
+
+
+def test_bench_rejects_zero_steps():
+    import subprocess
+    import sys
+    r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--steps', '0'], capture_output=True, text=True, timeout=120)
+    assert r.returncode != 0 and '--steps' in r.stderr
+
+
+def test_dump_outputs_samples_the_same_points_within_the_budget(tmp_path, monkeypatch):
+    import numpy as np
+    import bench
+    monkeypatch.setattr(bench, 'DUMP_BYTES', 64 << 10)
+    rng = np.random.default_rng(1)
+    arrays = {'type0': rng.random((4, 1024, 8, 1)), 'type1': rng.random((4, 1024, 8, 3)).astype(np.float16)}
+    for d in ('a', 'b'):
+        bench.dump_outputs(arrays, str(tmp_path / d))
+    got = {f: np.load(tmp_path / 'a' / f) for f in ('type0.npy', 'type1.npy')}
+    assert got['type0.npy'].dtype == np.float64 and got['type1.npy'].dtype == np.float32
+    assert sum(a.nbytes for a in got.values()) <= 64 << 10
+    rows0 = got['type0.npy'].reshape(len(got['type0.npy']), -1)
+    all0 = arrays['type0'].reshape(4096, -1)
+    assert len(rows0) > 1 and all(any((r == all0).all(1)) for r in rows0)       # whole rows of the output, not mixtures
+    for f, a in got.items():
+        assert np.array_equal(np.load(tmp_path / 'b' / f), a)
+
+
 def test_concurrent_builds_do_not_race(tmp_path):
     """One process per GPU: every rank may find the library missing at the same moment.  Three processes build a moved copy of
     the sources at once; the file lock lets one of them compile, the others wait and load the finished library (a rank once
