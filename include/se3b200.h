@@ -12,7 +12,7 @@
  *                                                                                               se3_pairwise_{simt,tc}_fwd
  *   masked_mean pooling of ConvSE3                     utils.py:72-80, S:256-257             -> se3_pool_fwd
  *   AttentionSE3.forward logits/softmax/aggregate      se3_transformer_pytorch.py:476-517    -> se3_attn_fwd
- *     (low-rank radial path: se3_pack_lowrank + se3_pairwise_lr_fwd / _strided_fwd, se3_fold_basis_fwd, se3_rotate_back_fwd:
+ *     (low-rank radial path: se3_pack_lowrank + se3_pairwise_lr_fwd, se3_fold_basis_fwd, se3_rotate_back_fwd:
  *      the same product re-associated; DESIGN.md 4.2-4.4)
  *   NormSE3.forward (next to the hot path, SURVEY 8f)  se3_transformer_pytorch.py:130-152    -> se3_norm_fwd
  *
@@ -113,13 +113,6 @@ int64_t se3_lowrank_image_bytes(int Co, int Ci, int F, int Kp);
 int se3_pack_lowrank(const float* Fp, int Co, int Ci, int F, int Kp, void* image, void* stream);
 int se3_pairwise_lr_fwd(const float* U, const void* w_img, const float* T, int64_t E, int Co, int Ci, int F, int P,
                         int Kp, int accumulate, float* out, void* stream);
-
-/* As se3_pairwise_lr_fwd, but component p of the kernel is written to out[e*edge_stride + o*channel_stride + p_off[p]]
- * (p_off: HOST array of P ints, P in {1,2,3,5,7}).  Used by the edge-aligned formulation (DESIGN.md 4.4), where one launch
- * updates the components (+m, -m) of a component-major [E, P_full, Co] buffer (channel_stride = 1). */
-int se3_pairwise_lr_strided_fwd(const float* U, const void* w_img, const float* T, int64_t E, int Co, int Ci, int F, int P,
-                                int Kp, int accumulate, float* out, int64_t edge_stride, int channel_stride, const int* p_off,
-                                void* stream);
 
 /* Basis fold of the input-side contraction (pairs with 2 l_in + 1 = Q < P = 2 l_out + 1; S:336-343, 251 reassociated):
  *   out[e,o,p] (+)= sum_{f,q} basis_pair[e,p,q,f] * S[f,e,o,q]

@@ -607,15 +607,6 @@ extern "C" int se3_pairwise_lr_fwd(const float* U, const void* w_img, const floa
   return pairwise_lr_impl(U, w_img, T, E, Co, Ci, F, P, Kp, accumulate, out, (int64_t)Co * P, P, nullptr, nullptr, stream);
 }
 
-// As se3_pairwise_lr_fwd, writing component p of the kernel to out[e*edge_stride + o*channel_stride + p_off[p]] (p_off: HOST
-// array of P ints): the edge-aligned formulation (DESIGN.md 4.4) updates two components (+m, -m) of a component-major
-// [E, P_full, Co] buffer per launch (channel_stride 1: every thread writes 8 consecutive floats per component).
-extern "C" int se3_pairwise_lr_strided_fwd(const float* U, const void* w_img, const float* T, int64_t E, int Co, int Ci, int F,
-                                           int P, int Kp, int accumulate, float* out, int64_t edge_stride, int channel_stride,
-                                           const int* p_off, void* stream) {
-  return pairwise_lr_impl(U, w_img, T, E, Co, Ci, F, P, Kp, accumulate, out, edge_stride, channel_stride, p_off, nullptr, stream);
-}
-
 // Diagnostic (tools/ only): same launch, and CTA 0 records clock64 stamps of its warp roles into trace[5][64][8].
 extern "C" int se3_pairwise_lr_trace(const float* U, const void* w_img, const float* T, int64_t E, int Co, int Ci, int F, int P,
                                      int Kp, int accumulate, float* out, unsigned long long* trace, void* stream) {

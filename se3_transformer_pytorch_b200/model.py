@@ -286,9 +286,10 @@ class ConvSE3(nn.Module):
         return torch.cat([xs.sin(), xs.cos(), rd], dim=-1)
 
     def lowrank_plan(self, d_max):
-        """Per pair: orthonormal V [128, r] spanning the curve g(d), d in [0, D], and the tensor-core image of
-        F'' = [W3 V | b3 | 0].  Depends on the weights and on D only: built once (and again if weights change or a forward
-        brings a larger distance).  Only for distance-only radial functions (no extra edge features)."""
+        """Per pair: orthonormal V [128, r] spanning the curve g(d), d in [0, D], and the tensor-core images of
+        F'' = [W3 V | b3 | 0] for the route the ConvSE3 will take.  Depends on the weights and on D only: built once (and again
+        if weights change or a forward brings a larger distance).  Only for distance-only radial functions (no extra edge
+        features)."""
         pk = self.packed()
         plan = pk.get('lr')
         if plan is not None and plan['D'] >= d_max:
@@ -297,83 +298,100 @@ class ConvSE3(nn.Module):
         D = 1.25 * d_max
         with torch.no_grad():
             grid = torch.linspace(0.0, D, self.LR_GRID, device=dev, dtype=torch.float64).unsqueeze(-1)
-            feat = self.encode_dist(grid)
-            pairs = {}
-            bases = {}
-            ugrid = {}
-            for di, do in self.pairs:
-                pc = self.kernel_unary[f'({di},{do})']
-                if self.tc_eligible(di, do) and pc.rp.net['6'].weight.numel() > 0:
-                    G64 = pc.rp.trunk64(feat)
-                    basis = ops.lowrank_basis(G64)
-                    if basis is not None:
-                        bases[(di, do)] = basis
-                        ugrid[(di, do)] = ((G64 - basis[2]) @ basis[1], float(G64.abs().max()))     # U(d) on the grid, float64
-                    del G64
+            bases, ugrid = self.lowrank_bases(grid)
+            covered = len(bases) == len(self.pairs)
             # the edge-aligned images serve a ConvSE3 only if EVERY pair has a plan (all launches of an output degree then
             # accumulate in the aligned frame); otherwise keep the global-frame images of 4.2-4.3 for the covered pairs
-            aligned_images = use_aligned() and len(bases) == len(self.pairs)
-            zplan = None
-            if aligned_images and use_zgemm() and self.zgemm_eligible({pair: 16 * ((rv[0] + 1 + 15) // 16) for pair, rv in bases.items()}):
-                zplan = {}                    # (do, m) -> dict(img, degs): one GEMM per output degree and |m| (DESIGN.md 4.5)
-                fps = {}
+            route = GLOBAL
+            if covered and use_aligned():
+                route = ZGEMM if use_zgemm() and self.zgemm_eligible({pair: _kp(r) for pair, (r, _, _) in bases.items()}) else ALIGNED
+            pairs, fps = {}, {}
             for (di, do), (r, V, gmean) in bases.items():
-                pc = self.kernel_unary[f'({di},{do})']
-                lin = pc.rp.net['6']
-                Kp = 16 * ((r + 1 + 15) // 16)
-                Fp = torch.zeros((lin.weight.shape[0], Kp), dtype=torch.float32, device=dev)
-                Fp[:, :r] = (lin.weight.double() @ V).float()
-                Fp[:, r] = (lin.bias.double() + lin.weight.double() @ gmean).float()      # affine model: W3 gmean joins the bias
-                Vp = torch.zeros((ops.RADIAL_MID, 64), dtype=torch.float32, device=dev)
-                Vp[:, :r] = V.float()
-                if zplan is not None:
-                    # the aligned weights w0, (a_m, b_m) = constant combinations of the F frequencies (rows (o,i,f) of F'); they are
-                    # concatenated over the input degrees into one GEMM image per (do, m) below
-                    Fv = Fp.view(pc.nc_out, pc.nc_in, pc.num_freq, Kp).double()
-                    c0, ca, cb = (t.to(dev) for t in _aligned.aligned_coeffs(di, do))
-                    fps[(di, do, 0)] = torch.einsum('oifk,f->oik', Fv, c0).reshape(-1, Kp).float().contiguous()
-                    for m in range(1, min(di, do) + 1):
-                        ab = torch.stack([torch.einsum('oifk,f->oik', Fv, ca[m - 1]), torch.einsum('oifk,f->oik', Fv, cb[m - 1])], dim=2)
-                        fps[(di, do, m)] = ab.reshape(-1, Kp).float().contiguous()
-                    pairs[(di, do)] = dict(r=r, Kp=Kp, V=Vp, gmean=gmean.float(), img=None, imgs_f=None, al_imgs=None, z=True)
-                    del Fv
-                elif aligned_images:
-                    # edge-aligned formulation (DESIGN.md 4.4): images of the weights a_m, b_m = constant combinations of the
-                    # F frequencies (rows (o,i,f) of F'), one image per m
-                    Fv = Fp.view(pc.nc_out, pc.nc_in, pc.num_freq, Kp).double()
-                    c0, ca, cb = (t.to(dev) for t in _aligned.aligned_coeffs(di, do))
-                    imgs = [ops.pack_lowrank(torch.einsum('oifk,f->oik', Fv, c0).reshape(-1, Kp).float().contiguous(),
-                                             pc.nc_out, pc.nc_in, 1, Kp)]
-                    for m in range(1, min(di, do) + 1):
-                        ab = torch.stack([torch.einsum('oifk,f->oik', Fv, ca[m - 1]), torch.einsum('oifk,f->oik', Fv, cb[m - 1])], dim=2)
-                        imgs.append(ops.pack_lowrank(ab.reshape(-1, Kp).float().contiguous(), pc.nc_out, pc.nc_in, 2, Kp))
-                    pairs[(di, do)] = dict(r=r, Kp=Kp, V=Vp, gmean=gmean.float(), img=None, imgs_f=None, al_imgs=imgs)
-                    del Fv
-                elif input_side(di, do) and pc.num_freq > 1:
-                    # input-side contraction (DESIGN.md 4.3): one image per frequency f (rows (o,i,f) of F'), no combined image
-                    Fv = Fp.view(pc.nc_out, pc.nc_in, pc.num_freq, Kp)
-                    imgs = [ops.pack_lowrank(Fv[:, :, f, :].reshape(-1, Kp).contiguous(), pc.nc_out, pc.nc_in, 1, Kp)
-                            for f in range(pc.num_freq)]
-                    pairs[(di, do)] = dict(r=r, Kp=Kp, V=Vp, gmean=gmean.float(), img=None, imgs_f=imgs)
+                Fp = self.fold_w3(di, do, r, V, gmean)
+                pairs[(di, do)] = rec = dict(r=r, Kp=_kp(r), V=torch.zeros((ops.RADIAL_MID, 64), dtype=torch.float32, device=dev),
+                                             gmean=gmean.float())
+                rec['V'][:, :r] = V.float()
+                if route == ZGEMM:               # concatenated over the input degrees into one GEMM image per (do, m) below
+                    fps.update({(di, do, m): w for m, w in enumerate(self.aligned_weights(di, do, Fp))})
+                elif route == ALIGNED:           # one image per |m| (DESIGN.md 4.4)
+                    pc = self.kernel_unary[f'({di},{do})']
+                    rec['al_imgs'] = [ops.pack_lowrank(w, pc.nc_out, pc.nc_in, 1 if m == 0 else 2, rec['Kp'])
+                                      for m, w in enumerate(self.aligned_weights(di, do, Fp))]
                 else:
-                    img = ops.pack_lowrank(Fp, pc.nc_out, pc.nc_in, pc.num_freq, Kp)
-                    pairs[(di, do)] = dict(r=r, Kp=Kp, V=Vp, gmean=gmean.float(), img=img, imgs_f=[img] if pc.num_freq == 1 else None)
+                    rec.update(self.global_images(di, do, Fp))
                 del Fp
-            if zplan is not None:
-                for do, mo in self.fiber_out:
-                    for m in range(do + 1):
-                        degs = [(di, mi) for di, mi in self.fiber_in if di >= m]
-                        if not degs:
-                            continue
-                        mode = 1 if m == 0 else z_mode_m()
-                        img, S = ops.zgemm_image([(fps.pop((di, do, m)), mi) for di, mi in degs], mo, mode)
-                        zplan[(do, m)] = dict(img=img, S=S, degs=degs, mode=mode)
-                del fps
-            utab = self.radial_table(ugrid, bases, grid, dev) if len(bases) == len(self.pairs) and use_utable() else None
-            del ugrid
-        plan = dict(D=D, pairs=pairs, z=zplan, utab=utab)
+            zplan = self.zgemm_images(fps) if route == ZGEMM else None
+            utab = self.radial_table(ugrid, bases, grid, dev) if covered and use_utable() else None
+            del ugrid, fps
+            # per-pair operands of the radial kernels, stacked over all pairs of the ConvSE3 (zero for pairs without a plan)
+            zero = torch.zeros((ops.RADIAL_MID, 64), dtype=torch.float32, device=dev)
+            recs = [pairs.get(p, dict(V=zero, gmean=zero[:, 0], r=0)) for p in self.pairs]
+            plan = dict(D=D, pairs=pairs, z=zplan, utab=utab, Vstack=torch.stack([p['V'] for p in recs]),
+                        gmean=torch.stack([p['gmean'] for p in recs]), ones_col=torch.tensor([p['r'] for p in recs], dtype=torch.int32, device=dev),
+                        have=torch.tensor([p in pairs for p in self.pairs], device=dev))
         pk['lr'] = plan
         return plan
+
+    def lowrank_bases(self, grid):
+        """{pair: (r, V, gmean)} low-rank bases of the trunk outputs on the grid, {pair: (U(d) on the grid, max|g|)}."""
+        feat = self.encode_dist(grid)
+        bases, ugrid = {}, {}
+        for di, do in self.pairs:
+            pc = self.kernel_unary[f'({di},{do})']
+            if self.tc_eligible(di, do) and pc.rp.net['6'].weight.numel() > 0:
+                G64 = pc.rp.trunk64(feat)
+                basis = ops.lowrank_basis(G64)
+                if basis is not None:
+                    bases[(di, do)] = basis
+                    ugrid[(di, do)] = ((G64 - basis[2]) @ basis[1], float(G64.abs().max()))     # U(d) on the grid, float64
+                del G64
+        return bases, ugrid
+
+    def fold_w3(self, di, do, r, V, gmean):
+        """F' = [W3 V | b3 + W3 gmean | 0] [Co*Ci*F, Kp] fp32, rows (o, i, f): the radial weights as a function of U."""
+        lin = self.kernel_unary[f'({di},{do})'].rp.net['6']
+        Fp = torch.zeros((lin.weight.shape[0], _kp(r)), dtype=torch.float32, device=V.device)
+        Fp[:, :r] = (lin.weight.double() @ V).float()
+        Fp[:, r] = (lin.bias.double() + lin.weight.double() @ gmean).float()      # affine model: W3 gmean joins the bias
+        return Fp
+
+    def aligned_weights(self, di, do, Fp):
+        """The edge-aligned weights w0, (a_m, b_m), m = 1..min(di, do): constant combinations of the F frequencies (rows
+        (o,i,f) of F'), as [Co*Ci, Kp] for m = 0 and [Co*Ci*2, Kp] (rows (o, i, (a, b))) otherwise."""
+        pc = self.kernel_unary[f'({di},{do})']
+        Kp = Fp.shape[1]
+        Fv = Fp.view(pc.nc_out, pc.nc_in, pc.num_freq, Kp).double()
+        c0, ca, cb = (t.to(Fp.device) for t in _aligned.aligned_coeffs(di, do))
+        out = [torch.einsum('oifk,f->oik', Fv, c0).reshape(-1, Kp).float().contiguous()]
+        for m in range(1, min(di, do) + 1):
+            ab = torch.stack([torch.einsum('oifk,f->oik', Fv, ca[m - 1]), torch.einsum('oifk,f->oik', Fv, cb[m - 1])], dim=2)
+            out.append(ab.reshape(-1, Kp).float().contiguous())
+        return out
+
+    def global_images(self, di, do, Fp):
+        """Global frame (DESIGN.md 4.2-4.3): `img` (all frequencies) for the output-side contraction, `imgs_f` (one per
+        frequency) for the input-side one; a single-frequency pair has both."""
+        pc = self.kernel_unary[f'({di},{do})']
+        Kp = Fp.shape[1]
+        if input_side(di, do) and pc.num_freq > 1:
+            Fv = Fp.view(pc.nc_out, pc.nc_in, pc.num_freq, Kp)
+            return dict(imgs_f=[ops.pack_lowrank(Fv[:, :, f, :].reshape(-1, Kp).contiguous(), pc.nc_out, pc.nc_in, 1, Kp)
+                                for f in range(pc.num_freq)])
+        img = ops.pack_lowrank(Fp, pc.nc_out, pc.nc_in, pc.num_freq, Kp)
+        return dict(img=img, imgs_f=[img]) if pc.num_freq == 1 else dict(img=img)
+
+    def zgemm_images(self, fps):
+        """{(do, m): one GEMM image over the input degrees di >= m (DESIGN.md 4.5)} from the aligned weights fps[(di, do, m)]."""
+        zplan = {}
+        for do, mo in self.fiber_out:
+            for m in range(do + 1):
+                degs = [(di, mi) for di, mi in self.fiber_in if di >= m]
+                if not degs:
+                    continue
+                mode = 1 if m == 0 else z_mode_m()
+                img, S = ops.zgemm_image([(fps.pop((di, do, m)), mi) for di, mi in degs], mo, mode)
+                zplan[(do, m)] = dict(img=img, S=S, degs=degs, mode=mode)
+        return zplan
 
     UTABLE_TOL = 5e-7        # max interpolation error of the tabulated radial coordinates relative to max|g| (float64, grid midpoints)
 
@@ -383,7 +401,7 @@ class ConvSE3(nn.Module):
         per edge.  Accepted only if the interpolant reproduces the float64 trunk at the grid MIDPOINTS to UTABLE_TOL (smooth
         radial functions pass by orders of magnitude; a rougher one falls back to se3_radial_trunk_u_fwd)."""
         Gn = grid.shape[0]
-        KT = max(16 * ((bases[p][0] + 1 + 15) // 16) for p in self.pairs)
+        KT = max(_kp(bases[p][0]) for p in self.pairs)
         tab = torch.zeros((len(self.pairs), Gn, KT), dtype=torch.float32, device=dev)
         mid = (grid[:-1] + grid[1:]) * 0.5
         featm = self.encode_dist(mid)
@@ -440,12 +458,7 @@ class ConvSE3(nn.Module):
     # ---- forward ----------------------------------------------------------------------------------------
     def edge_features(self, edge_info, rel_dist):
         _, _, edges = edge_info
-        rd = rel_dist.unsqueeze(-1)
-        if self.fourier_encode_dist:
-            # reference utils.py:96-104: [sin(x / 2^s), cos(x / 2^s), x]
-            scales = 2 ** torch.arange(self.num_fourier_features, device=rd.device, dtype=rd.dtype)
-            xs = rd / scales
-            rd = torch.cat([xs.sin(), xs.cos(), rd], dim=-1)
+        rd = self.encode_dist(rel_dist.unsqueeze(-1))
         feat = torch.cat((rd, edges), dim=-1) if exists(edges) else rd
         return feat.reshape(-1, feat.shape[-1]).contiguous()
 
@@ -500,10 +513,8 @@ class Geometry:
         if not isinstance(akv, AlignedKV):
             return akv
         b, n, k, P, C = akv.t.shape
-        E = b * n * k
-        out = torch.empty((E, C, P), dtype=torch.float32, device=akv.t.device)
-        ops.fold_basis(akv.t.reshape(1, E, P, C), self.frames().D[akv.lo].reshape(-1), E, C, P, P, 1, out, accumulate=False,
-                       component_major=True, name='rotate_back')
+        out = torch.empty((b * n * k, C, P), dtype=torch.float32, device=akv.t.device)
+        rotate_to_global(akv.t.reshape(-1, P, C), self.frames().D[akv.lo], out)
         return out.view(b, n, k, C, P)
 
     def frames(self):
@@ -544,175 +555,183 @@ class LowRankPlanMiss(RuntimeError):
     """The radial trunk outputs of a forward left the cached low-rank subspace (distances beyond the plan's range)."""
 
 
+ZGEMM, ALIGNED, GLOBAL = 'zgemm', 'aligned', 'global'       # the routes of a ConvSE3 forward (conv_route, DESIGN.md 4)
+
+
+def _kp(r):
+    """K of the low-rank radial GEMM: r basis columns + the ones column, in steps of 16."""
+    return 16 * ((r + 1 + 15) // 16)
+
+
+def conv_route(conv, E, edge_info, rel_dist, geom, capturing):
+    """The route of one ConvSE3 for this forward and what it needs: dict(route, lr = {pair: plan record} of the low-rank pairs,
+    U / g = outputs of the radial kernels it launches, z = the one-GEMM images, outs = per-edge output buffers)."""
+    pk = conv.packed()
+    feat = conv.edge_features(edge_info, rel_dist)
+    assert feat.shape[-1] == conv.in_dim, f'edge feature width {feat.shape[-1]} != {conv.in_dim}'
+    tc_ok = {pair: conv.tc_eligible(*pair) for pair in conv.pairs}
+    # low-rank radial path (distance-only radial functions): U = G V with the pair's cached basis, K = r+1 <= 64
+    plan = None
+    if os.environ.get('SE3B200_NO_LOWRANK') or conv.edge_dim != 0:
+        pass
+    elif conv.free_master and pk.get('lr') is not None:
+        plan = pk['lr']                         # built by pack_weights(max_distance=...) before the masters went away:
+                                                # the only image there is, whatever the edge count
+    elif ops.lowrank_enabled(E) and any(tc_ok.values()) and not conv.free_master and not getattr(conv, '_lr_blocked', False):
+        # while capturing: the plan the warm-up forwards built (the residual check below still covers it); otherwise cached,
+        # it needs the distance range (one host sync per forward, in Geometry)
+        plan = pk.get('lr') if capturing else conv.lowrank_plan(geom.d_max(rel_dist) if geom is not None else float(rel_dist.max()))
+    st = dict(conv=conv, route=GLOBAL, tc_ok=tc_ok, lr={}, U=None, g=None, z=None,
+              outs={do: torch.empty((E, mo, to_order(do)), dtype=torch.float32, device=feat.device) for do, mo in conv.fiber_out})
+    if plan is not None and plan['pairs']:
+        # trunk + U = G V + the residual statistics of the cached subspace on THIS forward's edges, one kernel
+        covered = len(plan['pairs']) == len(conv.pairs)
+        stats = torch.zeros((len(conv.pairs), 2), dtype=torch.float32, device=feat.device)
+        if covered and plan['utab'] is not None and use_utable():
+            # distance-only radial functions: U(d) interpolated from the plan's float64 table; the guard is the table's range
+            st['U'] = ops.radial_table(rel_dist, plan['utab'], plan['D'], plan['ones_col'], stats)
+        else:
+            st['U'], st['g'] = ops.radial_trunk_u(feat, pk['trunk'], plan['Vstack'], plan['gmean'], plan['ones_col'], stats,
+                                                  want_g=not covered)
+        st['lr'] = dict(plan['pairs'])
+        check = (conv, stats, plan['have'])
+        if geom is not None and geom.deferred is not None:
+            geom.deferred.append(check)          # checked once per forward by the caller
+        elif check_lowrank_stats([check]):
+            # the fp32 trunk outputs of this forward leave the cached subspace (distances beyond the plan's range)
+            if conv.free_master:
+                raise LowRankPlanMiss('low-rank radial plan does not cover this input; pack_weights(max_distance=...) was given too '
+                                      'small a distance')
+            st['lr'] = {}                        # evaluate this ConvSE3 with the direct K = 128 kernels
+        if st['lr'] and covered and geom is not None:
+            if plan['z'] is not None:
+                st['route'], st['z'] = ZGEMM, plan['z']
+            elif all('al_imgs' in pp for pp in st['lr'].values()):
+                st['route'] = ALIGNED
+    if st['route'] == GLOBAL and any('img' not in pp and 'imgs_f' not in pp for pp in st['lr'].values()):
+        # the plan holds edge-aligned images only (DESIGN.md 4.4-4.5); they need the per-forward Geometry
+        if geom is None:
+            raise RuntimeError('ConvSE3 was called with a (flat, plan) basis: the edge-aligned low-rank plan needs the third element, '
+                               'model.Geometry(rel_pos, max_degree), as SE3Transformer.forward passes it (or set SE3B200_NO_ALIGNED=1)')
+        st['lr'] = {}                            # images that do not fit this route: direct kernels for this forward
+    if st['route'] == GLOBAL and len(st['lr']) < len(conv.pairs) and st['g'] is None:
+        st['g'] = ops.radial_trunk(feat, pk['trunk'], len(conv.pairs))       # the direct kernels consume g itself
+    return st
+
+
+def edge_chunks(E, bytes_per_tile):
+    """[(first tile, tiles, first edge, edges)] of the edge chunks whose workspace fits T_WORKSPACE_BYTES."""
+    n_tiles = (E + ops.TILE_E - 1) // ops.TILE_E
+    per_chunk = max(1, min(n_tiles, T_WORKSPACE_BYTES // bytes_per_tile))
+    return [(t0, min(per_chunk, n_tiles - t0), t0 * ops.TILE_E, min(E - t0 * ops.TILE_E, per_chunk * ops.TILE_E))
+            for t0 in range(0, n_tiles, per_chunk)]
+
+
+def rotate_to_global(t, D, out):
+    """Edge-aligned outputs back to the global frame: out [E, C, P] = D(e) t[e], t [E, P, C] component major, D [E, P, P]."""
+    E, P, C = t.shape
+    ops.fold_basis(t.reshape(1, E, P, C), D.reshape(-1), E, C, P, P, 1, out, accumulate=False, component_major=True, name='rotate_back')
+
+
 def conv_forward(convs, inp, edge_info, rel_dist, basis, keep_aligned=False):
-    """Evaluate one or more ConvSE3 that share input features, graph and fibers (to_k / to_v of an attention block)
-    in a single sweep: the T blocks (gather x basis) are built once per (degree pair, edge chunk) and consumed by every
-    convolution's fused pairwise kernel."""
-    c0 = convs[0]
+    """Evaluate one or more ConvSE3 that share input features, graph and fibers (to_k / to_v of an attention block): each
+    takes its route (conv_route); the convolutions on one route share its per-chunk gathers."""
     forward_only_guard('ConvSE3', convs, list(inp.values()) + [rel_dist])
     idx, nmask, _ = edge_info
-    b, n, k = idx.shape
-    E = b * n * k
-    dev = idx.device
+    E = idx.numel()
     if isinstance(basis, dict):
         raise TypeError("ConvSE3 takes the basis as the tuple (flat buffer, BasisPlan, Geometry) that SE3Transformer.forward builds: "
                         "`ops.basis_flat(rel_pos, max_degree) + (model.Geometry(rel_pos, max_degree),)`; the dict returned by the "
                         "drop-in get_basis() is the reference's per-pair view of the same buffer and is not accepted here")
-    flat, plan = basis[:2]                   # BasisFlat (+ Geometry)
     geom = basis[2] if len(basis) > 2 else None
-    bpairs = ops.basis_pairs(flat, plan, E)
-    n_tiles = (E + ops.TILE_E - 1) // ops.TILE_E
-
-    states = []
     capturing = torch.cuda.is_current_stream_capturing()
+    states = []
     for conv in convs:
-        assert conv.pairs == c0.pairs and conv.in_dim == c0.in_dim
-        pk = conv.packed()
-        feat = conv.edge_features(edge_info, rel_dist)
-        assert feat.shape[-1] == conv.in_dim, f'edge feature width {feat.shape[-1]} != {conv.in_dim}'
-        tc_ok = {pair: conv.tc_eligible(*pair) for pair in conv.pairs}
-        # low-rank radial path (distance-only radial functions): U = G V with the pair's cached basis, K = r+1 <= 64
-        lr, lr_plan = {}, None
-        if os.environ.get('SE3B200_NO_LOWRANK') or conv.edge_dim != 0:
-            pass
-        elif conv.free_master and pk.get('lr') is not None:
-            lr_plan = pk['lr']                      # built by pack_weights(max_distance=...) before the masters went away:
-                                                    # the only image there is, whatever the edge count
-        elif ops.lowrank_enabled(E) and any(tc_ok.values()) and not conv.free_master and not getattr(conv, '_lr_blocked', False):
-            if capturing:
-                lr_plan = pk.get('lr')              # built by the warm-up forwards; the residual check below still covers it
-            else:                                   # cached; needs the distance range (one host sync per forward, in Geometry)
-                lr_plan = conv.lowrank_plan(geom.d_max(rel_dist) if geom is not None else float(rel_dist.max()))
-        g, U, zplan = None, None, None
-        if lr_plan is not None and lr_plan['pairs']:
-            if 'Vstack' not in lr_plan:
-                Vs = torch.zeros((len(conv.pairs), ops.RADIAL_MID, 64), dtype=torch.float32, device=dev)
-                gm = torch.zeros((len(conv.pairs), ops.RADIAL_MID), dtype=torch.float32, device=dev)
-                ones_col = torch.zeros(len(conv.pairs), dtype=torch.int32, device=dev)
-                have = torch.zeros(len(conv.pairs), dtype=torch.bool, device=dev)
-                for pi, pair in enumerate(conv.pairs):
-                    pp = lr_plan['pairs'].get(pair)
-                    if pp is not None:
-                        Vs[pi] = pp['V']
-                        gm[pi] = pp['gmean']
-                        ones_col[pi] = pp['r']
-                        have[pi] = True
-                lr_plan['Vstack'], lr_plan['gmean'], lr_plan['ones_col'], lr_plan['have'] = Vs, gm, ones_col, have
-            # trunk + U = G V + the residual statistics of the cached subspace on THIS forward's edges, one kernel
-            covered = len(lr_plan['pairs']) == len(conv.pairs)
-            stats = torch.zeros((len(conv.pairs), 2), dtype=torch.float32, device=dev)
-            if covered and lr_plan.get('utab') is not None and use_utable():
-                # distance-only radial functions: U(d) interpolated from the plan's float64 table; the guard is the table's range
-                U, g = ops.radial_table(rel_dist, lr_plan['utab'], lr_plan['D'], lr_plan['ones_col'], stats), None
-            else:
-                U, g = ops.radial_trunk_u(feat, pk['trunk'], lr_plan['Vstack'], lr_plan['gmean'], lr_plan['ones_col'], stats, want_g=not covered)
-            for pi, pair in enumerate(conv.pairs):
-                pp = lr_plan['pairs'].get(pair)
-                if pp is not None:
-                    lr[pair] = dict(Kp=pp['Kp'], U=U[pi], img=pp['img'], imgs_f=pp.get('imgs_f'), al_imgs=pp.get('al_imgs'))
-            check = (conv, stats, lr_plan['have'])
-            if geom is not None and geom.deferred is not None:
-                geom.deferred.append(check)          # checked once per forward by the caller
-            elif check_lowrank_stats([check]):
-                # the fp32 trunk outputs of this forward leave the cached subspace (distances beyond the plan's range)
-                if conv.free_master:
-                    raise LowRankPlanMiss('low-rank radial plan does not cover this input; pack_weights(max_distance=...) was given too '
-                                          'small a distance')
-                lr = {}                              # evaluate this ConvSE3 with the direct K = 128 kernel
-            if lr and covered and geom is not None:
-                zplan = lr_plan.get('z')
-        outs = {do: torch.empty((E, mo, to_order(do)), dtype=torch.float32, device=dev) for do, mo in conv.fiber_out}
-        al = zplan is None and geom is not None and len(lr) == len(conv.pairs) and all(v.get('al_imgs') is not None for v in lr.values())
-        if zplan is None and not al and any(v.get('img') is None and v.get('imgs_f') is None for v in lr.values()):
-            # the plan holds edge-aligned images only (DESIGN.md 4.4-4.5); they need the per-forward Geometry
-            if geom is None:
-                raise RuntimeError('ConvSE3 was called with a (flat, plan) basis: the edge-aligned low-rank plan needs the third element, '
-                                   'model.Geometry(rel_pos, max_degree), as SE3Transformer.forward passes it (or set SE3B200_NO_ALIGNED=1)')
-            lr = {}                                  # mixed eligibility inside one ConvSE3: direct kernels for this forward
-        if zplan is None and len(lr) < len(conv.pairs) and g is None:
-            g = ops.radial_trunk(feat, pk['trunk'], len(conv.pairs))       # the direct kernels consume g itself
-        states.append(dict(conv=conv, pk=pk, g=g, U=U, outs=outs, use_tc=tc_ok, lr=lr, aligned=al, z=zplan, lr_plan=lr_plan))
-    states_z_and_rest = list(states)            # in the order of `convs`
-    z_states = [st for st in states if st['z'] is not None]
-    states = [st for st in states if st['z'] is None]
-    if z_states:
-        # ---- production path (DESIGN.md 4.5): neighbour features rotated into the edge frame once per input degree, then ONE
-        # tensor-core GEMM per (conv, degree_out, |m|) over all input degrees, then the rotation back to the global frame
-        frames = geom.frames()
-        sx = ops.edge_scale(inp, idx, max(di for di, _ in c0.fiber_in))
-        per_tile = sum(mi * to_order(di) for di, mi in c0.fiber_in) * ops.TILE_E * 4
-        tpc = max(1, min(n_tiles, T_WORKSPACE_BYTES // per_tile))
-        # pooled convolutions (conv_in / conv_out): masked mean over the neighbours + self-interaction fused into the rotate-back
-        # (needs edge chunks that hold whole neighbour lists)
-        fuse_pool = tpc >= n_tiles or (tpc * ops.TILE_E) % k == 0
-        for st in z_states:
-            conv = st['conv']
-            if conv.pool and fuse_pool:
-                st['pooled'] = {do: torch.empty((b * n, mo, to_order(do)), dtype=torch.float32, device=dev) for do, mo in conv.fiber_out}
-                st['self'] = conv.self_interact(inp) if conv.self_interaction else {}
-        nmask_flat = None if nmask is None else nmask.reshape(-1)
-        for st in z_states:
-            if keep_aligned and 'pooled' not in st:      # the consumer (attention) rotates back on the fly: keep out' itself
-                st['aligned_out'] = {do: torch.empty((E, to_order(do), mo), dtype=torch.float32, device=dev)
-                                     for do, mo in st['conv'].fiber_out if do > 0}
-        for t0 in range(0, n_tiles, tpc):
-            tc = min(tpc, n_tiles - t0)
-            e0 = t0 * ops.TILE_E
-            ec = min(E - e0, tc * ops.TILE_E)
-            X = {di: ops.rotgather(inp[str(di)], idx, frames.D[di] if di > 0 else None, t0, tc) for di, _ in c0.fiber_in}
-            for st in z_states:
-                conv = st['conv']
-                for do, mo in conv.fiber_out:
-                    P = to_order(do)
-                    full = all((do, m) in st['z'] for m in range(do + 1))
-                    if do == 0 and 'pooled' not in st:
-                        Op = st['outs'][0][e0:e0 + ec]                   # [ec, mo, 1] is [ec, 1, mo]
-                    elif do in st.get('aligned_out', {}):
-                        Op = st['aligned_out'][do][e0:e0 + ec]
-                        if not full:
-                            Op.zero_()
-                    else:
-                        Op = (torch.empty if full else torch.zeros)((ec, P, mo), dtype=torch.float32, device=dev)
-                    for m in range(do + 1):
-                        zp = st['z'].get((do, m))
-                        if zp is None:
-                            continue
-                        segs, alg = [], 0
-                        for di, mi in zp['degs']:
-                            pi = conv.pairs.index((di, do))
-                            for kc in range(st['lr'][(di, do)]['Kp'] // 16):
-                                segs.append((st['U'][pi, e0:e0 + ec, 16 * kc:], X[di], mi, to_order(di), di + m, di - m))
-                            alg += ec * mo * mi * 2 * (ops.RADIAL_MID + P) * (1 if m == 0 else 2)
-                        ops.zgemm(segs, zp['img'], sx[e0:e0 + ec], ec, mo, zp['mode'], Op, P * mo, [(do + m) * mo, (do - m) * mo],
-                                  alg_flops=alg, tag=f'mode{zp["mode"]}lo{do}m{m}Co{mo}S{zp["S"]}')
-                    if 'pooled' in st:                  # rotate back + masked mean over k + self-interaction, one kernel
-                        sa = st['self'].get(str(do))
-                        ops.rotate_pool(Op, frames.D[do][e0:e0 + ec] if do > 0 else None, None if nmask_flat is None else nmask_flat[e0:e0 + ec],
-                                        None if sa is None else sa.reshape(b * n, mo, P)[e0 // k:(e0 + ec) // k], ec // k, k, mo, do,
-                                        st['pooled'][do][e0 // k:(e0 + ec) // k])
-                    elif do in st.get('aligned_out', {}):
-                        pass                            # stays in the edge frame; rotated inside the attention kernel
-                    elif do > 0:                        # back to the global frame: out = D_lo out'
-                        ops.fold_basis(Op.view(1, ec, P, mo), frames.D[do][e0:e0 + ec].reshape(-1), ec, mo, P, P, 1,
-                                       st['outs'][do][e0:e0 + ec], accumulate=False, component_major=True, name='rotate_back')
-            del X
-    aligned_states = [st for st in states if st['aligned']]
-    states_all, states = states_z_and_rest, [st for st in states if not st['aligned']]
+        assert conv.pairs == convs[0].pairs and conv.in_dim == convs[0].in_dim
+        states.append(conv_route(conv, E, edge_info, rel_dist, geom, capturing))
+    routed = {route: [st for st in states if st['route'] == route] for route in (ZGEMM, ALIGNED, GLOBAL)}
+    if routed[ZGEMM]:
+        eval_zgemm(routed[ZGEMM], inp, idx, nmask, geom, keep_aligned)
+    workspace = eval_aligned(routed[ALIGNED], inp, idx, geom) if routed[ALIGNED] else None
+    if routed[GLOBAL]:
+        eval_global(routed[GLOBAL], inp, idx, ops.basis_pairs(basis[0], basis[1], E), workspace)
+    return [conv_outputs(st, inp, idx, nmask) for st in states]
 
-    # chunk over edge tiles so that the largest T block fits the workspace
-    worst = max(ops.t_numel(1, mi, to_order(min(di, do)), to_order(do)) * 4
-                for di, mi in c0.fiber_in for do, _ in c0.fiber_out)
-    tiles_per_chunk = max(1, min(n_tiles, T_WORKSPACE_BYTES // worst))
+
+def eval_zgemm(states, inp, idx, nmask, geom, keep_aligned):
+    """Production path (DESIGN.md 4.5): neighbour features rotated into the edge frame once per input degree and chunk, then
+    ONE tensor-core GEMM per (conv, degree_out, |m|) over all input degrees, then the rotation back to the global frame."""
+    c0 = states[0]['conv']
+    b, n, k = idx.shape
+    E, dev = b * n * k, idx.device
+    frames = geom.frames()
+    sx = ops.edge_scale(inp, idx, max(di for di, _ in c0.fiber_in))
+    chunks = edge_chunks(E, sum(mi * to_order(di) for di, mi in c0.fiber_in) * ops.TILE_E * 4)
+    # pooled convolutions (conv_in / conv_out): masked mean over the neighbours + self-interaction fused into the rotate-back
+    # (needs edge chunks that hold whole neighbour lists)
+    fuse_pool = len(chunks) == 1 or (chunks[0][1] * ops.TILE_E) % k == 0
+    for st in states:
+        conv = st['conv']
+        if conv.pool and fuse_pool:
+            st['pooled'] = {do: torch.empty((b * n, mo, to_order(do)), dtype=torch.float32, device=dev) for do, mo in conv.fiber_out}
+            st['self'] = conv.self_interact(inp) if conv.self_interaction else {}
+        elif keep_aligned:                          # the consumer (attention) rotates back on the fly: keep out' itself
+            st['aligned_out'] = {do: torch.empty((E, to_order(do), mo), dtype=torch.float32, device=dev) for do, mo in conv.fiber_out if do > 0}
+    nmask_flat = None if nmask is None else nmask.reshape(-1)
+    for t0, tc, e0, ec in chunks:
+        X = {di: ops.rotgather(inp[str(di)], idx, frames.D[di] if di > 0 else None, t0, tc) for di, _ in c0.fiber_in}
+        for st in states:
+            conv = st['conv']
+            for do, mo in conv.fiber_out:
+                P = to_order(do)
+                full = all((do, m) in st['z'] for m in range(do + 1))
+                if do == 0 and 'pooled' not in st:
+                    Op = st['outs'][0][e0:e0 + ec]                   # [ec, mo, 1] is [ec, 1, mo]
+                elif do in st.get('aligned_out', {}):
+                    Op = st['aligned_out'][do][e0:e0 + ec]
+                    if not full:
+                        Op.zero_()
+                else:
+                    Op = (torch.empty if full else torch.zeros)((ec, P, mo), dtype=torch.float32, device=dev)
+                for m in range(do + 1):
+                    zp = st['z'].get((do, m))
+                    if zp is None:
+                        continue
+                    segs, alg = [], 0
+                    for di, mi in zp['degs']:
+                        pi = conv.pairs.index((di, do))
+                        for kc in range(st['lr'][(di, do)]['Kp'] // 16):
+                            segs.append((st['U'][pi, e0:e0 + ec, 16 * kc:], X[di], mi, to_order(di), di + m, di - m))
+                        alg += ec * mo * mi * 2 * (ops.RADIAL_MID + P) * (1 if m == 0 else 2)
+                    ops.zgemm(segs, zp['img'], sx[e0:e0 + ec], ec, mo, zp['mode'], Op, P * mo, [(do + m) * mo, (do - m) * mo],
+                              alg_flops=alg, tag=f'mode{zp["mode"]}lo{do}m{m}Co{mo}S{zp["S"]}')
+                if 'pooled' in st:                  # rotate back + masked mean over k + self-interaction, one kernel
+                    sa = st['self'].get(str(do))
+                    ops.rotate_pool(Op, frames.D[do][e0:e0 + ec] if do > 0 else None, None if nmask_flat is None else nmask_flat[e0:e0 + ec],
+                                    None if sa is None else sa.reshape(b * n, mo, P)[e0 // k:(e0 + ec) // k], ec // k, k, mo, do,
+                                    st['pooled'][do][e0 // k:(e0 + ec) // k])
+                elif do > 0 and do not in st.get('aligned_out', {}):    # (aligned_out stays in the edge frame for the attention kernel)
+                    rotate_to_global(Op, frames.D[do][e0:e0 + ec], st['outs'][do][e0:e0 + ec])
+        del X
+
+
+def tbuild_chunks(conv, E):
+    """Edge chunks in which the largest T block of the R-first kernels fits the workspace."""
+    return edge_chunks(E, max(ops.t_numel(1, mi, to_order(min(di, do)), to_order(do)) * 4
+                              for di, mi in conv.fiber_in for do, _ in conv.fiber_out))
+
+
+def eval_aligned(states, inp, idx, geom):
+    """R-first edge-aligned formulation (DESIGN.md 4.4): neighbour features rotated into the edge frame per (degree_in, |m|)
+    and chunk, two output components per launch, then the rotation back.  Returns the T workspace."""
+    c0 = states[0]['conv']
+    E, dev = idx.numel(), idx.device
     workspace = None
-    for t0 in range(0, n_tiles, tiles_per_chunk) if aligned_states else ():
-        # ---- edge-aligned formulation: rotate the neighbour features into the edge frame, two output components per launch
-        tc = min(tiles_per_chunk, n_tiles - t0)
-        e0 = t0 * ops.TILE_E
-        ec = min(E - e0, tc * ops.TILE_E)
+    for t0, tc, e0, ec in tbuild_chunks(c0, E):
         frames = geom.frames()
         # out' of degree do lives in one dense buffer per |m|: [edges, C_out] for m = 0, [edges, C_out, 2] = (+m, -m) otherwise
         # (the kernel's native layout); first contribution overwrites, later input degrees accumulate
-        outp = [{} for _ in aligned_states]
+        outp = [{} for _ in states]
         for di, mi in c0.fiber_in:
             for m in range(di + 1):
                 targets = [(do, mo) for do, mo in c0.fiber_out if do >= m]
@@ -721,15 +740,15 @@ def conv_forward(convs, inp, edge_info, rel_dist, basis, keep_aligned=False):
                 Pk = Fk = 1 if m == 0 else 2
                 workspace = ops.tbuild_blocks(inp[str(di)], idx, frames.block(di, m), Pk, Fk, t0, tc, out=workspace)
                 for do, mo in targets:
-                    P = to_order(do)
-                    for st, op in zip(aligned_states, outp):
+                    pi = c0.pairs.index((di, do))
+                    for st, op in zip(states, outp):
                         lrp = st['lr'][(di, do)]
                         first = (do, m) not in op
                         if first:
                             op[(do, m)] = st['outs'][do][e0:e0 + ec] if do == 0 else torch.empty((ec, mo, Pk), dtype=torch.float32, device=dev)
-                        ops.pairwise_lr(lrp['U'][e0:e0 + ec], lrp['al_imgs'][m], workspace, ec, mo, mi, Fk, Pk, lrp['Kp'], op[(do, m)],
-                                        accumulate=not first, alg_units=Fk * 2 * (ops.RADIAL_MID + P))
-        for st, op in zip(aligned_states, outp):
+                        ops.pairwise_lr(st['U'][pi, e0:e0 + ec], lrp['al_imgs'][m], workspace, ec, mo, mi, Fk, Pk, lrp['Kp'], op[(do, m)],
+                                        accumulate=not first, alg_units=Fk * 2 * (ops.RADIAL_MID + to_order(do)))
+        for st, op in zip(states, outp):
             for do, mo in c0.fiber_out:
                 if do > 0:                      # back to the global frame: out = D_lo out'
                     ops.rotate_back([op.get((do, m)) for m in range(do + 1)], frames.D[do][e0:e0 + ec].reshape(-1), ec, mo, do,
@@ -737,10 +756,15 @@ def conv_forward(convs, inp, edge_info, rel_dist, basis, keep_aligned=False):
                 elif (0, 0) not in op:
                     st['outs'][0][e0:e0 + ec].zero_()
         del outp
-    for t0 in range(0, n_tiles, tiles_per_chunk) if states else ():
-        tc = min(tiles_per_chunk, n_tiles - t0)
-        e0 = t0 * ops.TILE_E
-        ec = min(E - e0, tc * ops.TILE_E)
+    return workspace
+
+
+def eval_global(states, inp, idx, bpairs, workspace=None):
+    """Per pair in the global frame (DESIGN.md 4.1-4.3): T = gather x basis once per (pair, chunk), then per convolution the
+    low-rank kernel (output- or input-side contraction) or the direct K = 128 kernel."""
+    c0 = states[0]['conv']
+    E, dev = idx.numel(), idx.device
+    for t0, tc, e0, ec in tbuild_chunks(c0, E):
         gathered = {}                            # degree_in -> neighbour features of this chunk in tile layout
         for do, mo in c0.fiber_out:
             P = to_order(do)
@@ -748,7 +772,7 @@ def conv_forward(convs, inp, edge_info, rel_dist, basis, keep_aligned=False):
             for di, mi in c0.fiber_in:
                 Fq = to_order(min(di, do))
                 Q = to_order(di)
-                in_side = [input_side(di, do) and (di, do) in st['lr'] and st['lr'][(di, do)]['imgs_f'] is not None for st in states]
+                in_side = [input_side(di, do) and 'imgs_f' in st['lr'].get((di, do), {}) for st in states]
                 if any(in_side) and di not in gathered:
                     gathered[di] = ops.gather_tiles(inp[str(di)], idx, t0, tc)
                 if not all(in_side):
@@ -762,16 +786,16 @@ def conv_forward(convs, inp, edge_info, rel_dist, basis, keep_aligned=False):
                         lrp = st['lr'][(di, do)]
                         S = torch.empty((Fq, ec, mo, Q), dtype=torch.float32, device=dev)
                         for f in range(Fq):
-                            ops.pairwise_lr(lrp['U'][e0:e0 + ec], lrp['imgs_f'][f], gathered[di], ec, mo, mi, 1, Q, lrp['Kp'], S[f],
+                            ops.pairwise_lr(st['U'][pi, e0:e0 + ec], lrp['imgs_f'][f], gathered[di], ec, mo, mi, 1, Q, lrp['Kp'], S[f],
                                             accumulate=False, alg_P=P)
                         ops.fold_basis(S, bpairs[(di, do)][e0 * P * Q * Fq:(e0 + ec) * P * Q * Fq], ec, mo, P, Q, Fq, out,
                                        accumulate=not first)
                         del S
                     elif (di, do) in st['lr']:
                         lrp = st['lr'][(di, do)]
-                        ops.pairwise_lr(lrp['U'][e0:e0 + ec], lrp['img'], workspace, ec, mo, mi, Fq, P, lrp['Kp'], out,
+                        ops.pairwise_lr(st['U'][pi, e0:e0 + ec], lrp['img'], workspace, ec, mo, mi, Fq, P, lrp['Kp'], out,
                                         accumulate=not first)
-                    elif st['use_tc'][(di, do)]:
+                    elif st['tc_ok'][(di, do)]:
                         ops.pairwise_tc(st['g'][pi, e0:e0 + ec], conv.w3_image(di, do), workspace, ec, mo, mi, Fq, P,
                                         out, accumulate=not first)
                     else:
@@ -780,25 +804,23 @@ def conv_forward(convs, inp, edge_info, rel_dist, basis, keep_aligned=False):
                                           accumulate=not first)
                 first = False
 
-    results = []
-    for st in states_all:
-        conv = st['conv']
-        outputs = {}
-        if 'pooled' in st:
-            results.append({str(do): st['pooled'][do].view(b, n, mo, to_order(do)) for do, mo in conv.fiber_out})
+
+def conv_outputs(st, inp, idx, nmask):
+    """The result of one ConvSE3: pooled, AlignedKV or per-edge outputs, plus the self-interaction residual."""
+    conv = st['conv']
+    b, n, k = idx.shape
+    if 'pooled' in st:
+        return {str(do): st['pooled'][do].view(b, n, mo, to_order(do)) for do, mo in conv.fiber_out}
+    outputs = {}
+    for do, mo in conv.fiber_out:
+        if do in st.get('aligned_out', {}):
+            outputs[str(do)] = AlignedKV(st['aligned_out'][do].view(b, n, k, to_order(do), mo), do)
             continue
-        for do, mo in conv.fiber_out:
-            if do in st.get('aligned_out', {}):
-                outputs[str(do)] = AlignedKV(st['aligned_out'][do].view(b, n, k, to_order(do), mo), do)
-                continue
-            o = st['outs'][do].view(b, n, k, mo, to_order(do))
-            if conv.pool:
-                o = ops.pool(o, nmask)
-            outputs[str(do)] = o
-        if conv.self_interaction:
-            outputs = residual_add(outputs, conv.self_interact(inp))
-        results.append(outputs)
-    return results
+        o = st['outs'][do].view(b, n, k, mo, to_order(do))
+        outputs[str(do)] = ops.pool(o, nmask) if conv.pool else o
+    if conv.self_interaction:
+        outputs = residual_add(outputs, conv.self_interact(inp))
+    return outputs
 
 
 class FeedForwardSE3(nn.Module):

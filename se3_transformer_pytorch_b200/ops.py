@@ -35,7 +35,6 @@ _SIGNATURES = {
     'se3_lowrank_image_bytes': (c_int64, [c_int, c_int, c_int, c_int]),
     'se3_pack_lowrank': (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     'se3_pairwise_lr_fwd': (c_int, [c_void_p] * 3 + [c_int64] + [c_int] * 6 + [c_void_p, c_void_p]),
-    'se3_pairwise_lr_strided_fwd': (c_int, [c_void_p] * 3 + [c_int64] + [c_int] * 6 + [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     'se3_pairwise_lr_trace': (c_int, [c_void_p] * 3 + [c_int64] + [c_int] * 6 + [c_void_p, c_void_p, c_void_p]),
     'se3_fold_basis_fwd': (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     'se3_fold_basis_cm_fwd': (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
@@ -444,7 +443,7 @@ def pack_lowrank(Fp, Co, Ci, F, Kp):
     return img
 
 
-def pairwise_lr(U, w_img, T, E, Co, Ci, F, P, Kp, out, accumulate, alg_P=None, out_strides=None, p_off=None, alg_units=None):
+def pairwise_lr(U, w_img, T, E, Co, Ci, F, P, Kp, out, accumulate, alg_P=None, alg_units=None):
     """Low-rank radial path: U [E,64] fp32 (G V | 1 | 0), w_img from pack_lowrank."""
     _require_cuda(U, w_img, T, out)
     # algorithmic work of the reference formulation (SURVEY.md 8d): 2*128 (radial GEMM) + 2P (contraction) per R element;
@@ -459,12 +458,7 @@ def pairwise_lr(U, w_img, T, E, Co, Ci, F, P, Kp, out, accumulate, alg_P=None, o
     tag = f'P{P}F{F}Ci{Ci}Co{Co}K{Kp}' + (f'(in-side of P{alg_P})' if alg_P is not None else '')
     with torch.cuda.device(out.device), _timed('pairwise_lr', flops=flops, nbytes=nbytes, tag=tag,
                                                mma=2 * E * Co * Ci * F * 3 * Kp, fma=2 * E * Co * Ci * F * P):
-        if out_strides is None:
-            _check(lib().se3_pairwise_lr_fwd(_p(U), _p(w_img), _p(T), E, Co, Ci, F, P, Kp, int(accumulate), _p(out), _stream()))
-        else:
-            offs = (ctypes.c_int * P)(*p_off)
-            _check(lib().se3_pairwise_lr_strided_fwd(_p(U), _p(w_img), _p(T), E, Co, Ci, F, P, Kp, int(accumulate), _p(out),
-                                                     out_strides[0], out_strides[1], offs, _stream()))
+        _check(lib().se3_pairwise_lr_fwd(_p(U), _p(w_img), _p(T), E, Co, Ci, F, P, Kp, int(accumulate), _p(out), _stream()))
 
 
 # ---------------------------------------------------------------------------------------------------------

@@ -126,221 +126,6 @@ def test_aligned_frames_reproduce_the_reference_basis():
             assert np.abs(pred - ref).max() < 2e-6 * max(1.0, np.abs(ref).max()), (li, lo)
 
 
-def test_lowrank_plan_image_selection(monkeypatch):
-    """Host logic of ConvSE3.lowrank_plan on CPU (the CUDA packer is stubbed): distance-only radial trunks factor with rank
-    <= 31, every pair of an all-eligible ConvSE3 gets edge-aligned images (one per |m|, F = 1 or 2 weight columns), a
-    ConvSE3 with an ineligible pair keeps the global-frame images for the pairs it does cover."""
-    import torch
-    from se3_transformer_pytorch_b200 import ops, model as M
-    calls = []
-
-    def fake_pack(Fp, Co, Ci, F, Kp):
-        assert Fp.shape == (Co * Ci * F, Kp) and Fp.dtype == torch.float32 and Fp.is_contiguous()
-        calls.append((Co, Ci, F, Kp))
-        return torch.zeros(1)
-
-    monkeypatch.setattr(ops, 'pack_lowrank', fake_pack)
-    monkeypatch.delenv('SE3B200_NO_ALIGNED', raising=False)
-    torch.manual_seed(0)
-    fin, fout = M.Fiber([(0, 32), (1, 32), (2, 32)]), M.Fiber([(0, 32), (1, 32), (2, 32)])
-    monkeypatch.setattr(M.ConvSE3, 'tc_eligible', lambda self, di, do: True)
-    conv = M.ConvSE3(fin, fout, edge_dim=0, pool=False, self_interaction=False)
-    plan = conv.lowrank_plan(4.0)
-    assert set(plan['pairs']) == set(conv.pairs)
-    for (di, do), pp in plan['pairs'].items():
-        assert pp['r'] <= 31 and pp['Kp'] in (16, 32)
-        assert pp['img'] is None and pp['imgs_f'] is None and len(pp['al_imgs']) == 1 + min(di, do)
-    assert sorted(c[2] for c in calls) == [1] * 9 + [2] * 5          # 9 pairs: one m = 0 image each; sum of min(di,do) = 5
-    calls.clear()
-    monkeypatch.setattr(M.ConvSE3, 'tc_eligible', lambda self, di, do: (di, do) != (2, 2))
-    conv2 = M.ConvSE3(fin, fout, edge_dim=0, pool=False, self_interaction=False)
-    plan2 = conv2.lowrank_plan(4.0)
-    assert (2, 2) not in plan2['pairs'] and len(plan2['pairs']) == 8
-    assert all(pp.get('al_imgs') is None and (pp['img'] is not None or pp['imgs_f'] is not None) for pp in plan2['pairs'].values())
-    assert conv2.lowrank_plan(3.0) is plan2                          # cached while the distance range is covered
-
-
-@pytest.mark.parametrize('frame', ['zgemm', 'aligned', 'global'])
-def test_lowrank_conv_dispatch_on_cpu_emulation(monkeypatch, frame):
-    """conv_forward's low-rank dispatch -- the one-GEMM production path (DESIGN.md 4.5: rotated gather, K segments per input
-    degree and 16-column block of U, component planes, rotate-back), the R-first edge-aligned path (4.4) and the global frame
-    with input-side contraction (4.2-4.3) (plan images, per-(l_in, m) tiles, (+m,-m) buffers, rotate-back, edge chunking)
-    with every CUDA op replaced by a float64 torch emulation of its contract, against the reference order of operations
-    (kernel = R . B first, S:336-343, with the oracle's basis).  Host logic only: the CUDA kernels have their own GPU tests."""
-    import numpy as np
-    import torch
-    from oracle import se3_oracle as O
-    from se3_transformer_pytorch_b200 import ops, model as M
-
-    torch.manual_seed(0)
-    b, n, k, C = 1, 40, 8, (128 if frame == 'zgemm' else 32)      # the one-GEMM kernel takes C_out % 128 == 0
-    L = 2
-    fin, fout = M.Fiber([(d, C) for d in range(L + 1)]), M.Fiber([(d, C) for d in range(L + 1)])
-    if frame in ('aligned', 'zgemm'):
-        monkeypatch.delenv('SE3B200_NO_ALIGNED', raising=False)
-    else:
-        monkeypatch.setenv('SE3B200_NO_ALIGNED', '1')
-    monkeypatch.delenv('SE3B200_NO_ZGEMM', raising=False)
-    monkeypatch.setenv('SE3B200_HOST_FRAMES', '1')               # float64 torch frames (the device kernel has its own GPU test)
-    monkeypatch.setattr(M.ConvSE3, 'tc_eligible', lambda self, di, do: True)
-    monkeypatch.setattr(ops, 'lowrank_enabled', lambda E: True)
-    monkeypatch.setattr(torch.cuda, 'is_current_stream_capturing', lambda: False)
-    monkeypatch.setattr(M, 'T_WORKSPACE_BYTES', ops.t_numel(1, C, 2, 2) * 4 if frame != 'zgemm' else 9 * C * ops.TILE_E * 4)  # one edge tile per chunk -> 3 chunks
-    monkeypatch.setattr(ops, 'pack_lowrank', lambda Fp, Co, Ci, F, Kp: Fp.double().clone())  # "image" = F' itself
-
-    conv = M.ConvSE3(fin, fout, edge_dim=0, pool=False, self_interaction=False)
-
-    def radial_trunk(feat, params, num_pairs):
-        return torch.stack([conv.kernel_unary[f'({di},{do})'].rp.trunk64(feat.double()) for di, do in conv.pairs]).float()
-
-    def radial_trunk_u(feat, params, V, gmean, ones_col, stats, want_g=False):
-        g = radial_trunk(feat, params, len(conv.pairs)).double()
-        gc = g - gmean.double()[:, None, :]
-        U = torch.bmm(gc, V.double())
-        resid = (gc - torch.bmm(U, V.double().transpose(1, 2))).abs().amax(dim=(1, 2))
-        stats[:, 0] = torch.maximum(stats[:, 0], resid.float())
-        stats[:, 1] = torch.maximum(stats[:, 1], g.abs().amax(dim=(1, 2)).float())
-        U[torch.arange(len(conv.pairs)), :, ones_col.long()] = 1.0
-        return U.float(), (g.float() if want_g else None)
-
-    def radial_table(dist, table, Dmax, ones_col, stats):
-        # float64 restatement of se3_radial_table_fwd: 4-point Lagrange interpolation of the plan's U(d) table
-        d = dist.reshape(-1).double()
-        assert float(d.max()) <= Dmax
-        Gn, KT = table.shape[1], table.shape[2]
-        t = d * (Gn - 1) / Dmax
-        i0 = t.floor().long().clamp(1, Gn - 3)
-        f = (t - i0).unsqueeze(-1)
-        w = (-f * (f - 1) * (f - 2) / 6, (f + 1) * (f - 1) * (f - 2) / 2, -(f + 1) * f * (f - 2) / 2, (f + 1) * f * (f - 1) / 6)
-        U = torch.zeros(table.shape[0], d.numel(), 64, dtype=torch.float64)
-        U[:, :, :KT] = sum(w[j] * table.double()[:, i0 - 1 + j] for j in range(4))
-        U[torch.arange(table.shape[0]), :, ones_col.long()] = 1.0
-        return U.float()
-
-    def rotgather(x, idx, D, tile_begin=0, tile_count=None, out=None):
-        E = idx.numel()
-        e0, e1 = tile_begin * ops.TILE_E, min(E, (tile_begin + tile_count) * ops.TILE_E)
-        xj = gather_rows(x, idx, e0, e1)
-        return xj if D is None else torch.einsum('eqn,eiq->ein', D[e0:e1].double(), xj)      # x'[n] = sum_q D[q,n] x[q]
-
-    def edge_scale(feats, idx, max_degree):
-        return torch.full((idx.numel(),), 4.0)
-
-    def zgemm_image(parts, Co, mode):
-        per_seg = (lambda Ci: 3 * (Ci // 4)) if mode == 3 else (lambda Ci: Ci * min(mode, 2) // 4)
-        return [(Fp.double(), Ci) for Fp, Ci in parts], sum((Fp.shape[1] // 16) * per_seg(Ci) for Fp, Ci in parts)
-
-    launched = []
-
-    def zgemm(segs, w_img, sx, E, Co, mode, out, out_edge_stride, comp_off, flush_stages=0, alg_flops=0, tag=''):
-        launched.append(tag)
-        mode = min(mode, 2)                                    # mode 3 = mode 2 evaluated with three products per complex one
-        assert out_edge_stride == out.shape[1] * out.shape[2] and sx.shape == (E,)
-        planes = out.view(E, -1, Co)                           # component-major rows: plane index = comp_off / Co
-        res = [torch.zeros(E, Co, dtype=torch.float64) for _ in range(mode)]
-        si = 0
-        for Fp, Ci in w_img:
-            Kp = Fp.shape[1]
-            Fv = Fp.reshape(Co, Ci, mode, Kp)
-            for kc in range(Kp // 16):
-                U, X, Ci_s, ncomp, cplus, cminus = segs[si]
-                si += 1
-                assert Ci_s == Ci and X.shape == (E, Ci, ncomp) and U.shape[0] == E
-                w = torch.einsum('ek,oifk->eoif', U[:, :16].double(), Fv[..., 16 * kc:16 * kc + 16])
-                if mode == 1:
-                    res[0] += torch.einsum('eoi,ei->eo', w[..., 0], X[:, :, cplus])
-                else:
-                    a, bb_ = w[..., 0], w[..., 1]
-                    res[0] += torch.einsum('eoi,ei->eo', a, X[:, :, cplus]) - torch.einsum('eoi,ei->eo', bb_, X[:, :, cminus])
-                    res[1] += torch.einsum('eoi,ei->eo', bb_, X[:, :, cplus]) + torch.einsum('eoi,ei->eo', a, X[:, :, cminus])
-        assert si == len(segs)
-        for c in range(mode):
-            planes[:, comp_off[c] // Co, :] = res[c].float()
-
-    def tbuild_blocks(x, idx, blocks, P, F, tile_begin=0, tile_count=None, out=None):
-        bb, nn, Ci, Q = x.shape
-        E = idx.numel()
-        e0, e1 = tile_begin * ops.TILE_E, min(E, (tile_begin + tile_count) * ops.TILE_E)
-        xj = x.reshape(bb * nn, Ci, Q)[(idx + torch.arange(bb).view(-1, 1, 1) * nn).reshape(-1)][e0:e1].double()
-        blk = blocks.reshape(E, P, Q, F)[e0:e1].double()
-        return torch.einsum('epqf,eiq->eifp', blk, xj)                             # T[e,i,f,p]
-
-    def gather_rows(x, idx, e0, e1):
-        bb, nn, Ci, Q = x.shape
-        return x.reshape(bb * nn, Ci, Q)[(idx + torch.arange(bb).view(-1, 1, 1) * nn).reshape(-1)][e0:e1].double()
-
-    def tbuild(x, idx, basis_pair, d_in, d_out, tile_begin=0, tile_count=None, out=None):
-        E = idx.numel()
-        P, Q, F = 2 * d_out + 1, 2 * d_in + 1, 2 * min(d_in, d_out) + 1
-        e0, e1 = tile_begin * ops.TILE_E, min(E, (tile_begin + tile_count) * ops.TILE_E)
-        return torch.einsum('epqf,eiq->eifp', basis_pair.reshape(E, P, Q, F)[e0:e1].double(), gather_rows(x, idx, e0, e1))
-
-    def gather_tiles(x, idx, tile_begin=0, tile_count=None, out=None):
-        E = idx.numel()
-        e0, e1 = tile_begin * ops.TILE_E, min(E, (tile_begin + tile_count) * ops.TILE_E)
-        return gather_rows(x, idx, e0, e1).unsqueeze(2)                             # [e, i, f = 1, q]
-
-    def fold_basis(S, basis_pair, E, Co, P, Q, F, out, accumulate, component_major=False, name='fold_basis'):
-        res = torch.einsum('epqf,feqo->eop' if component_major else 'epqf,feoq->eop', basis_pair.reshape(E, P, Q, F).double(), S.double())
-        out.copy_((out.double() + res if accumulate else res).float())
-
-    def pairwise_lr(U, img, T, E, Co, Ci, F, P, Kp, out, accumulate, alg_P=None, out_strides=None, p_off=None, alg_units=None):
-        assert out_strides is None and T.shape == (E, Ci, F, P) and out.shape[0] == E
-        R = (U[:, :Kp].double() @ img.t()).reshape(E, Co, Ci, F)                    # bias rides on the ones column of U
-        res = torch.einsum('eoif,eifp->eop', R, T).reshape(out.shape)
-        out.copy_((out.double() + res if accumulate else res).float())
-
-    def rotate_back(parts, D, E, Co, lo, out):
-        P = 2 * lo + 1
-        v = torch.zeros((E, Co, P), dtype=torch.float64)
-        if parts[0] is not None:
-            v[:, :, lo] = parts[0].reshape(E, Co).double()
-        for m in range(1, lo + 1):
-            if parts[m] is not None:
-                v[:, :, lo + m], v[:, :, lo - m] = parts[m][:, :, 0].double(), parts[m][:, :, 1].double()
-        out.copy_(torch.einsum('epn,eon->eop', D.reshape(E, P, P).double(), v).float())
-
-    for name, fn in (('radial_trunk', radial_trunk), ('tbuild_blocks', tbuild_blocks), ('pairwise_lr', pairwise_lr),
-                     ('rotate_back', rotate_back), ('tbuild', tbuild), ('gather_tiles', gather_tiles), ('fold_basis', fold_basis),
-                     ('radial_trunk_u', radial_trunk_u), ('radial_table', radial_table), ('rotgather', rotgather), ('edge_scale', edge_scale), ('zgemm_image', zgemm_image),
-                     ('zgemm', zgemm)):
-        monkeypatch.setattr(ops, name, fn)
-
-    coors = torch.randn(b, n, 3)
-    idx = torch.stack([torch.randperm(n - 1)[:k] for _ in range(b * n)]).reshape(b, n, k)
-    idx = idx + (idx >= torch.arange(n).view(1, n, 1)).long()                        # neighbours != self
-    rel_pos = coors[0][:, None, :] - coors[0][idx[0]]                                # x_i - x_j   (S:1222)
-    rel_pos = rel_pos.reshape(b, n, k, 3)
-    rel_dist = rel_pos.norm(dim=-1)
-    inp = {str(d): torch.randn(b, n, C, 2 * d + 1) for d in range(L + 1)}
-
-    E = b * n * k
-    Bo = O.get_basis(rel_pos.reshape(E, 3).double().numpy(), L)
-    monkeypatch.setattr(ops, 'basis_pairs', lambda flat, plan, E_: {(di, do): torch.from_numpy(np.asarray(Bo[f'{di},{do}'])).reshape(-1)
-                                                                     for di in range(L + 1) for do in range(L + 1)})
-    basis = (torch.zeros(0), None, M.Geometry(rel_pos, L))
-    nmask = torch.ones(b, n, k, dtype=torch.bool)
-    with torch.no_grad():
-        out = M.conv_forward([conv], inp, (idx, nmask, None), rel_dist, basis)[0]
-
-    assert (len(launched) == 3 * (1 + 2 + 3)) == (frame == 'zgemm')       # 3 edge chunks x one launch per (degree_out, |m|)
-    # reference order of operations in float64
-    feat = rel_dist.reshape(E, 1).double()
-    worst = 0.0
-    for do in range(L + 1):
-        ref = np.zeros((E, C, 2 * do + 1))
-        for di in range(L + 1):
-            pc = conv.kernel_unary[f'({di},{do})']
-            lin = pc.rp.net['6']
-            g = pc.rp.trunk64(feat)
-            R = (g @ lin.weight.double().t() + lin.bias.double()).reshape(E, C, C, pc.num_freq).detach().numpy()
-            xj = inp[str(di)].reshape(n, C, 2 * di + 1)[idx.reshape(-1)].double().numpy()
-            ref += np.einsum('eoif,epqf,eiq->eop', R, np.asarray(Bo[f'{di},{do}']), xj)
-        got = out[str(do)].reshape(E, C, 2 * do + 1).numpy()
-        worst = max(worst, float(np.abs(got - ref).max() / np.abs(ref).max()))
-    assert worst < 2e-5, worst
-
-
 def _run_bench(extra, env=None):
     import json
     import subprocess
